@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SoftRas forward+backward throughput on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c2|tiny]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c2|tiny] [--dump-outputs DIR]
     (N>1: python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
 
 Workload (default "c3", BASELINE.json configs[2] / the README's 39k-face row): UV sphere with
@@ -28,6 +28,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only; nothing is written into it
 
 METRIC = "softras_fwd_bwd_frames_per_s_1024px_39k_faces"
 WORKLOADS = {
@@ -60,7 +61,24 @@ def parse_args():
     ap.add_argument("--option", action="append", default=[], metavar="NAME=VALUE",
                     help="b200r_set_option() knob for A/B runs, e.g. --option softras_exact_tail=1")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU-baseline sample time")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy")
     return ap.parse_args()
+
+
+DUMP_SAMPLE = 1 << 22   # elements kept of a larger output: at most 16 MiB of float32 per array, 64 MiB for four arrays
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each output as out_dir/<name>.npy (float32).  An output with more than DUMP_SAMPLE elements is replaced by
+    the elements at a fixed seeded sample of flat positions, so that two builds can be compared value for value."""
+    assert len(arrays) <= 4
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32)
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -150,6 +168,7 @@ def _run_json(cmd, timeout):
     env = dict(os.environ)
     for k in ("OMP_NUM_THREADS", "OMP_PROC_BIND", "OMP_PLACES"):   # torchrun exports OMP_NUM_THREADS=1
         env.pop(k, None)
+    env["PYTHONDONTWRITEBYTECODE"] = "1"
     try:
         r = subprocess.run([sys.executable] + cmd, cwd=ROOT, env=env, capture_output=True, text=True, timeout=timeout)
         for line in reversed(r.stdout.strip().splitlines()):
@@ -259,12 +278,16 @@ def run_ours(args, rank, world, local_rank):
     for a, b in ev:
         flush.fill_(1.0)          # L2 flush between timed iterations (outside the event pair)
         a.record()
-        step()
+        img = step()
         b.record()
     barrier()
     launches = L.b200r_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     step_ms = [a.elapsed_time(b) for a, b in ev]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"soft_colors": img.detach().cpu().numpy(), "grad_face_vertices": fv.grad.cpu().numpy(),
+                                         "grad_textures": tex.grad.cpu().numpy()})
+    del img
     t_rank = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t_rank, op=dist.ReduceOp.MAX)
@@ -607,7 +630,7 @@ def run_nmr(args, rank, world, local_rank):
     tex_h = np.ascontiguousarray(np.repeat(tex_h, bpg, 0))
     faces = torch.from_numpy(faces_h).to(dev).requires_grad_(True)
     tex = torch.from_numpy(tex_h).to(dev).requires_grad_(True)
-    g = torch.rand((bpg, H, H, 3), device=dev) * 2 - 1
+    g = torch.from_numpy(np.random.default_rng(3 + rank).uniform(-1.0, 1.0, (bpg, H, H, 3)).astype(np.float32)).to(dev)
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)
 
     def step():
@@ -615,6 +638,7 @@ def run_nmr(args, rank, world, local_rank):
         tex.grad = None
         rgb, _, _ = RasterizeFunction(H, 0.1, 100.0, 1e-3, (0, 0, 0), True, False, False)(faces, tex)
         rgb.backward(g)
+        return rgb
     for _ in range(max(3, args.warmup)):
         step()
     torch.cuda.synchronize(dev)
@@ -622,10 +646,14 @@ def run_nmr(args, rank, world, local_rank):
     l0 = L.b200r_launch_count()
     for a, b in ev:
         flush.fill_(1.0)
-        a.record(); step(); b.record()
+        a.record(); rgb = step(); b.record()
     torch.cuda.synchronize(dev)
     launches = L.b200r_launch_count() - l0
     ms = [a.elapsed_time(b) for a, b in ev]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"rgb": rgb.detach().cpu().numpy(), "grad_faces": faces.grad.cpu().numpy(),
+                                         "grad_textures": tex.grad.cpu().numpy()})
+    del rgb
     L.b200r_profile_reset(); L.b200r_profile_enable(1)
     for _ in range(3):
         flush.fill_(1.0); step()
@@ -735,6 +763,8 @@ def run_render(args, rank, world, local_rank):
     wall = time.perf_counter() - t0
     launches = L.b200r_launch_count() - l0
     ms = [a.elapsed_time(b) for a, b in ev]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"rgb": host.numpy()})
     L.b200r_profile_reset(); L.b200r_profile_enable(1)
     for k in range(5):
         frame(4.0 * k)
@@ -763,6 +793,9 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "c5"):
+        raise SystemExit("bench.py: --dump-outputs covers --impl ours on every workload but c5 (its loop runs inside "
+                         "examples/demo2_deform.py)")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

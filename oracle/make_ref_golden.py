@@ -11,6 +11,10 @@ tests/test_golden.py compares the CPU oracle to them on every run.
 Each .npz holds the inputs (face_vertices, textures, upstream gradient), the parameters, and
 the reference kernels' outputs (soft_colors, aggrs_info, faces_id_buffer, faces_info,
 grad_faces, grad_textures), plus the nvcc flags and GPU the reference was run with.
+
+--large-only writes refsample_*.npz instead: stratified samples of the reference outputs at C3 / C4 sizes for the
+GPU tests that compare the product with the reference there (tests/util.py).  It runs the product too, so the
+product library must be built.
 """
 import json
 import os
@@ -180,11 +184,47 @@ def bake_n3mr_main(out_dir):
         print(json.dumps(dict(name=name, max_abs_vs_oracle=float(np.abs(ref - cpu).max()))), flush=True)
 
 
+# Fixtures of the GPU tests that compare the product with the reference kernels at sizes the CPU oracle cannot reach
+# (test_softras_gpu.py::test_against_reference_kernels_on_gpu, test_nmr_gpu.py::test_c4_against_reference_kernels_on_gpu).
+# Whole outputs are tens of MB there, so a stratified sample is kept (tests/util.py:softras_fixture, nmr_fixture); the
+# strata follow where the product built from this tree disagrees with the reference, so build it first.
+# Sample sizes per fixture: the estimates must sit well inside the tests' tolerances over resampling (measured on a
+# B200 over 30 seeds).  39 200 faces at 1024^2 puts grad_faces at 0.097 against a bound of 0.10, so the 2048 faces
+# that carry most of that difference are all kept; NMR gradients sit 100x inside their bounds.
+LARGE_SOFTRAS = {(3280, 512): dict(n_pixels=1024, n_worst_faces=512, n_faces=512),
+                 (39200, 512): dict(n_pixels=1024, n_worst_faces=512, n_faces=512),
+                 (39200, 1024): dict(n_pixels=2048, n_worst_faces=2048, n_faces=1024)}
+SAMPLE_C4 = dict(n_pixels=2048, n_worst_faces=256, n_faces=256)
+
+
+def large_main(out_dir):
+    import torch
+    from tests import util
+    prov = lambda src: json.dumps(dict(gpu=torch.cuda.get_device_name(0), source=src + " via oracle/build_ref.py",   # noqa: E731
+                                       nvcc="12.9 -O3 -gencode arch=compute_100a,code=sm_100a (fmad default on)"))
+    for (nf, H), sample in LARGE_SOFTRAS.items():
+        fv, tex, g = util.large_softras_inputs(nf, H)
+        P = osr.Params(image_size=H)
+        ref, got = ref_gpu.run(fv, tex, P, grad=g), util.run_cuda(fv, tex, P, grad=g, want_faces_info=False)
+        np.savez_compressed(os.path.join(out_dir, "refsample_softras_%d_%d.npz" % (nf, H)), input_sums=util.input_sums(fv, tex, g),
+                            provenance=prov("jrender/renderer/dr/softras/cuda/soft_rasterize.py kernels"),
+                            **util.softras_fixture(ref, got, **sample))
+    faces, tex, g, ga = util.c4_inputs()
+    args = (faces, tex, 1024, 0.1, 100.0, 1e-3, (0, 0, 0), (True, True, False), (g, ga, None))
+    ref, got = ref_gpu.nmr_run(*args), util.run_nmr_cuda(*args)
+    np.savez_compressed(os.path.join(out_dir, "refsample_nmr_c4_1024.npz"), input_sums=util.input_sums(faces, tex, g, ga),
+                        provenance=prov("jrender/renderer/dr/n3mr/cuda/rasterize.py kernels"),
+                        **util.nmr_fixture(ref, got, far=100.0, **SAMPLE_C4))
+
+
 def main():
     import torch
     out_dir = os.path.join("gpurun_out", "golden")
     os.makedirs(out_dir, exist_ok=True)
     report = []
+    if "--large-only" in sys.argv:
+        large_main(out_dir)
+        return
     if "--bake-only" in sys.argv:
         bake_main(out_dir)
         bake_n3mr_main(out_dir)

@@ -5,7 +5,9 @@ Tolerances: bake vs the numpy oracle 2e-6 absolute (same formulas unfused on bot
 reference's own kernel on a B200 (tests/golden/ref_gpu_bake_random40_R5.npz) 1e-5 (its build contracts a*b+c).
 C1: top-K ids bit-exact, colours 2e-6, gradients 2e-5 of max -- the SoftRas parity bar (tests/test_softras_gpu.py).
 """
+import lzma
 import os
+import shutil
 
 import numpy as np
 import pytest
@@ -18,7 +20,19 @@ from oracle import softras as osr
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 G = os.path.join(ROOT, "tests", "golden")
-SPOT = os.path.join(ROOT, "baseline", "_ref", "assets", "data", "obj", "spot", "spot_triangulated.obj")
+
+
+@pytest.fixture(scope="module")
+def spot(tmp_path_factory):
+    """The reference's spot cow (data/obj/spot: OBJ + MTL + texture PNG), kept xz-compressed under tests/golden/spot and
+    unpacked next to its material files; returns the OBJ's path."""
+    d = tmp_path_factory.mktemp("spot")
+    src = os.path.join(G, "spot")
+    with lzma.open(os.path.join(src, "spot_triangulated.obj.xz")) as f, open(d / "spot_triangulated.obj", "wb") as g:
+        shutil.copyfileobj(f, g)
+    for name in ("spot_triangulated.mtl", "spot_texture.png"):
+        shutil.copyfile(os.path.join(src, name), d / name)
+    return str(d / "spot_triangulated.obj")
 
 
 def test_bake_kernel_matches_oracle_and_reference_kernel(cuda_device):
@@ -84,29 +98,27 @@ def test_n3mr_bake_kernel_matches_reference_kernel_golden(cuda_device):
             assert (d > 1e-5).mean() <= 2e-3, p
 
 
-@pytest.mark.skipif(not os.path.exists(SPOT), reason="reference assets not staged (python -m tools.stage_assets where /root/reference exists)")
-def test_n3mr_loader_bakes_the_spot_texture(cuda_device):
+def test_n3mr_loader_bakes_the_spot_texture(cuda_device, spot):
     """load_obj(dr_type='n3mr', load_texture=True) as demo4 would call it: [nf, ts, ts, ts, 3] textures whose baked texels
     equal the oracle's bake of the same image / UVs."""
     from jrender_b200 import io as jio
-    v, f, t = jio.load_obj(SPOT, load_texture=True, dr_type='n3mr', texture_res=4)
+    v, f, t = jio.load_obj(spot, load_texture=True, dr_type='n3mr', texture_res=4)
     assert tuple(t.shape) == (5856, 4, 4, 4, 3) and tuple(f.shape) == (5856, 3)
-    faces_uv, names = jio._parse_texture_faces(SPOT)
-    image = jio._imread_rgb01(os.path.join(os.path.dirname(SPOT), "spot_texture.png"))[::-1]
+    faces_uv, names = jio._parse_texture_faces(spot)
+    image = jio._imread_rgb01(os.path.join(os.path.dirname(spot), "spot_texture.png"))[::-1]
     ref = obake.bake_textures_for_n3mr(np.ascontiguousarray(image), faces_uv, np.full((5856, 4, 4, 4, 3), 0.5, np.float32),
                                        np.ones(5856, np.int32), 0, True)
     assert np.abs(t.numpy() - ref).max() <= 2e-6
     assert float(t.std()) > 0.05
 
 
-@pytest.mark.skipif(not os.path.exists(SPOT), reason="reference assets not staged (python -m tools.stage_assets where /root/reference exists)")
-def test_spot_through_the_nmr_renderer_against_oracle(cuda_device):
+def test_spot_through_the_nmr_renderer_against_oracle(cuda_device, spot):
     """The textured cow through Renderer(dr_type='n3mr') (demo4's renderer): loader + ts^3 bake + lighting + transform +
     N3mrRasterizer; the rasterizer's inputs are taken from the pipeline and handed to the NMR oracle, whose rgb map the
     returned image must equal bit for bit (after the host side's transpose and vertical flip, n3mr.py:239-247)."""
     from oracle import nmr as onmr
     from jrender_b200.n3mr import vertices_to_faces
-    mesh = jr.Mesh.from_obj(SPOT, load_texture=True, texture_res=4, dr_type='n3mr').to(cuda_device)
+    mesh = jr.Mesh.from_obj(spot, load_texture=True, texture_res=4, dr_type='n3mr').to(cuda_device)
     assert tuple(mesh.textures.shape) == (1, 5856, 4, 4, 4, 3)
     renderer = jr.Renderer(dr_type='n3mr', image_size=256, anti_aliasing=False)
     renderer.transform.set_eyes_from_angles(2.732, 30, 40)
@@ -124,12 +136,11 @@ def test_spot_through_the_nmr_renderer_against_oracle(cuda_device):
     assert 0.05 < float((img.sum(1) > 0).float().mean()) < 0.6 and float(img.std()) > 0.05
 
 
-@pytest.mark.skipif(not os.path.exists(SPOT), reason="reference assets not staged (python -m tools.stage_assets where /root/reference exists)")
-def test_c1_spot_render_as_demo1_against_oracle(cuda_device):
+def test_c1_spot_render_as_demo1_against_oracle(cuda_device, spot):
     """demo1-render.py: Mesh.from_obj(load_texture=True, texture_res=5) -> Renderer(dr_type='softras') -> render_mesh('rgb').
     The rasterizer's inputs (projected face vertices, lit T=25 textures) are taken from the pipeline and handed to the
     CPU oracle; forward compared in full, backward on every 16th row."""
-    mesh = jr.Mesh.from_obj(SPOT, load_texture=True, texture_res=5, texture_type='surface', dr_type='softras').to(cuda_device)
+    mesh = jr.Mesh.from_obj(spot, load_texture=True, texture_res=5, texture_type='surface', dr_type='softras').to(cuda_device)
     assert mesh.faces.shape[1] == 5856 and tuple(mesh.textures.shape) == (1, 5856, 25, 3)
     renderer = jr.Renderer(dr_type='softras')
     renderer.transform.set_eyes_from_angles(2.732, 30, 0)
@@ -163,18 +174,17 @@ def test_c1_spot_render_as_demo1_against_oracle(cuda_device):
     assert tex_leaf.grad is not None and float(tex_leaf.grad.abs().max()) > 0
 
 
-@pytest.mark.skipif(not os.path.exists(SPOT), reason="reference assets not staged (python -m tools.stage_assets where /root/reference exists)")
-def test_demo4_texture_optimisation_converges(cuda_device):
+def test_demo4_texture_optimisation_converges(cuda_device, spot):
     """examples/demo4_optim_textures.py (port of the reference's demo4: NMR renderer, orthogonal camera, ambient light, Adam on
     a [1, nf, 4, 4, 4, 3] texture parameter): 60 iterations against a render of the cow's own baked texture must cut the
     sum-of-squares loss by more than half; and the reference's own loader call (texture_res left at 1) must not fail."""
     import warnings
     from examples import demo4_optim_textures as d4
-    model, losses = d4.run(SPOT, None, iters=60, device=str(cuda_device))
+    model, losses = d4.run(spot, None, iters=60, device=str(cuda_device))
     assert np.isfinite(losses).all() and losses[-1] < 0.5 * losses[0], (losses[0], losses[-1])
     g = model.textures.grad
     assert g is not None and float(g.abs().max()) > 0
     with warnings.catch_warnings(record=True) as w:
         warnings.simplefilter("always")
-        m = jr.Mesh.from_obj(SPOT, dr_type='n3mr', load_texture=True)   # demo4-optim_textures.py:24
+        m = jr.Mesh.from_obj(spot, dr_type='n3mr', load_texture=True)   # demo4-optim_textures.py:24
         assert tuple(m.textures.shape) == (1, 5856, 1, 1, 1, 3) and any("texture_res" in str(x.message) for x in w)
