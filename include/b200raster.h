@@ -20,6 +20,9 @@
  *   b200r_nmr_backward      <- jrender/renderer/dr/n3mr/cuda/rasterize.py:342-648, :650-727,
  *                              :729-822 (backward_pixel_map, backward_textures,
  *                              backward_depth_map), called from n3mr.py:29-67.
+ *   b200r_sss_blur_chain    <- jrender/renderer/utils/ToStretchMap.py and the 36 _blur_for_SSS ops
+ *                              (renderer/utils/gaussian_blur.py:34-165) of SSS(), called from
+ *                              jrender/renderer/lighting/lighting.py:86-156 (Mesh.with_SSS).
  *
  * Conventions
  *   - All tensor pointers are DEVICE pointers owned by the caller (contiguous, fp32 /
@@ -251,6 +254,26 @@ B200R_API int b200r_surface_lighting_backward(const float* vertices, const int32
                                               float directional_intensity, const float* directional_color, const float* direction,
                                               int with_specular, void* stream);
 
+/* ---- texture-space subsurface scattering (Mesh.with_SSS) ------------------------------------------------------
+ * b200r_sss_blur_chain replaces the image-space part of SSS() (jrender/renderer/lighting/lighting.py:86-156): the stretch
+ * map of renderer/utils/ToStretchMap.py (of worldcoord * 7, clamped to [0, 1]) and the 36 launches of the stretch-modulated
+ * 7-tap Gaussian blur _blur_for_SSS (renderer/utils/gaussian_blur.py:34-165) for the variances 25, 75, 300, the weighted
+ * sum of the three basis images, `* irradiance + specular` and the vertical flip, in seven launches.
+ *   worldcoord_map, irradiance_map, specular_map  [>=3, S, S] planar (soft_colors of a texture-space rasterization)
+ *   final_map      [S, S, 3] out, flipped vertically, ready for b200r_bake_textures_softras
+ *   workspace      b200r_sss_workspace_bytes(S) bytes of device scratch (13 planes of S x S floats)
+ *   taps           HOST float[3][7]: Gauss[i] = sqrt(v) * N(v, -sqrt(v) * (3 - i)) per variance, computed in double and
+ *                  rounded to float (gaussian_blur.py:8-10); gauss_widths HOST float[3] = sqrt(v)
+ *   weights        HOST float[3][3]: weights[channel][basis] (R 0.7 0.2 0.1, G and B 0.1 0.2 0.7 in the reference)
+ * b200r_sss_blur is one _blur_for_SSS launch on a single S x S map: dim 1 blurs along x, dim 0 along y; taps HOST
+ * float[7].  Both keep the reference's FFMA contraction of the tap interpolation and accumulation (csrc/sss_api.cu). */
+B200R_API size_t b200r_sss_workspace_bytes(int image_size);
+B200R_API int b200r_sss_blur_chain(const float* worldcoord_map, const float* irradiance_map, const float* specular_map,
+                                   float* final_map, void* workspace, size_t workspace_bytes, int image_size,
+                                   const float* taps, const float* gauss_widths, const float* weights, void* stream);
+B200R_API int b200r_sss_blur(const float* image, const float* modulate, float* out, int image_size, const float* taps,
+                             float gauss_width, int dim, void* stream);
+
 B200R_API unsigned long long b200r_launch_count(void);
 
 /* Tuning knobs (process-wide; results are identical for every setting except softras_exact_tail):
@@ -269,7 +292,7 @@ enum { B200R_K_FACE_SETUP = 0, B200R_K_COARSE_BIN = 1, B200R_K_SOFTRAS_FWD = 2, 
        B200R_K_TILE_ORDER = 4, B200R_K_NMR_SETUP = 5, B200R_K_NMR_FWD = 6, B200R_K_NMR_BWD_PIXEL = 7,
        B200R_K_NMR_BWD_MAPS = 8, B200R_K_SOFTRAS_BWD_FINALIZE = 9, B200R_K_NMR_PACK = 10,
        B200R_K_PROJECT_FWD = 11, B200R_K_PROJECT_BWD = 12, B200R_K_FLATTEN_LOSS = 13, B200R_K_LAPLACIAN_LOSS = 14,
-       B200R_K_LIGHTING = 15, B200R_K_BAKE = 16 };
+       B200R_K_LIGHTING = 15, B200R_K_BAKE = 16, B200R_K_SSS = 17 };
 B200R_API void b200r_profile_enable(int on);
 B200R_API void b200r_profile_reset(void);
 B200R_API int b200r_profile_read(int kernel, double* total_ms, long long* launches);

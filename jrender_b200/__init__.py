@@ -10,7 +10,7 @@ from .softras import SoftRasterizeFunction, SoftRasterizer, soft_rasterize  # no
 from .mesh import Mesh, face_vertices, join_meshes_as_scene  # noqa: F401
 from .transform import (Transform, LookAt, Look, Projection, look_at, look, perspective, orthogonal,  # noqa: F401
                         projection, get_points_from_angles)
-from .lighting import Lighting, AmbientLighting, DirectionalLighting  # noqa: F401
+from .lighting import Lighting, AmbientLighting, DirectionalLighting, SSS  # noqa: F401
 from .renderer import Renderer  # noqa: F401
 from .preraster import project_faces  # noqa: F401
 from .loss import neg_iou_loss, LaplacianLoss, FlattenLoss  # noqa: F401

@@ -81,6 +81,12 @@ def lib():
     L.b200r_bake_textures_softras.argtypes = [_P, _P, _P, _P, _I, _I, _I, _I, _P]
     L.b200r_bake_textures_n3mr.restype = _I
     L.b200r_bake_textures_n3mr.argtypes = [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]
+    L.b200r_sss_workspace_bytes.restype = C.c_size_t
+    L.b200r_sss_workspace_bytes.argtypes = [_I]
+    L.b200r_sss_blur_chain.restype = _I
+    L.b200r_sss_blur_chain.argtypes = [_P] * 5 + [C.c_size_t, _I, _P, _P, _P, _P]
+    L.b200r_sss_blur.restype = _I
+    L.b200r_sss_blur.argtypes = [_P, _P, _P, _I, _P, _F, _I, _P]
     L.b200r_set_option.restype = _I
     L.b200r_set_option.argtypes = [C.c_char_p, _I]
     _lib = L

@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libb200raster.so")
 SOURCES = ["softras_api.cu", "softras_fwd.cu", "softras_bwd.cu",
-           "nmr_api.cu", "preraster_api.cu", "mesh_loss_api.cu", "lighting_api.cu", "bake_api.cu", "api_util.cu", "debug_api.cu"]
+           "nmr_api.cu", "preraster_api.cu", "mesh_loss_api.cu", "lighting_api.cu", "bake_api.cu", "sss_api.cu", "api_util.cu", "debug_api.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 OBJDIR = os.path.join(HERE, "lib", "obj")

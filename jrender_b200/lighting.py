@@ -4,10 +4,11 @@
 Mirrors jrender/renderer/lighting/{ambient_lighting,directional_lighting,lighting}.py for the
 paths the rasterizer demos use: ambient + directional light in 'surface' and 'vertex' modes,
 including the Cook-Torrance specular branch the reference takes by default
-(Mesh.with_specular defaults to True, structures/mesh.py:74).  Normal-mapped meshes
-(surface_ResNormals), SSS and the Gbuffer debug modes are not mirrored.
+(Mesh.with_specular defaults to True, structures/mesh.py:74), and texture-space subsurface scattering
+(Mesh.with_SSS, SSS below).  Normal-mapped meshes (surface_ResNormals) and the Gbuffer debug modes are not mirrored.
 """
 import ctypes as C
+import math
 
 import torch
 from torch import nn
@@ -167,6 +168,108 @@ class _FusedSurfaceLighting(torch.autograd.Function):
         return gv, (gt if ctx.needs_input_grad[1] else None), None, None, None, None, None
 
 
+_SSS_BASIS = [0, 25, 100, 400]                                          # lighting.py:115
+_SSS_WEIGHTS = [[0.7, 0.2, 0.1], [0.1, 0.2, 0.7], [0.1, 0.2, 0.7]]      # lighting.py:126-129, [channel][basis]
+_SSS_TAP_NUM = 7
+
+
+def _sss_taps(v):
+    """gaussian_blur.py:4-10 in double: the 7 taps and GaussWidth = sqrt(v) of one variance.  Both are rounded to float
+    on the way to the kernel, as in the reference (float32 tap tensor; jt.float32(GaussWidth) formatted into the launch)."""
+    w = math.sqrt(v)
+    return [w * (math.exp(-(-w * ((_SSS_TAP_NUM - 1) / 2 - k)) ** 2 / (2 * v)) / math.sqrt(2 * math.pi * v))
+            for k in range(_SSS_TAP_NUM)], w
+
+
+def _sss_host_arrays():
+    """Taps (3 x 7), Gauss widths (3) and weights (3 x 3) of the blur chain as host float arrays."""
+    taps, widths = [], []
+    for i in range(len(_SSS_BASIS) - 1):
+        t, w = _sss_taps(_SSS_BASIS[i + 1] - _SSS_BASIS[i])
+        taps += t
+        widths.append(w)
+    return ((C.c_float * len(taps))(*taps), (C.c_float * 3)(*widths),
+            (C.c_float * 9)(*[x for row in _SSS_WEIGHTS for x in row]))
+
+
+def SSS(diffuseLight, specular, mesh, image_size=2048):
+    """Texture-space subsurface scattering (lighting.py:86-156) of a softras mesh with 4-D textures and face_texcoords.
+
+    diffuseLight, specular: the per-face surface lighting terms [1, nf, 1, 3].  The mesh's world-space geometry, the
+    irradiance sqrt(textures * diffuseLight) and the specular term are rasterized into UV space at image_size^2; the
+    stretch-modulated Gaussian blur chain (b200r_sss_blur_chain) turns them into the scattered colour map, which is
+    baked back into textures [1, nf, texture_res^2, 3] (not clamped; Lighting clamps).
+
+    The result is DETACHED: the reference's blur and bake ops have no gradient, so neither have these textures.
+    Batch 1 only, like the reference (it squeezes the batch axis)."""
+    from .io import bake_textures_for_softras
+    from .softras import SoftRasterizeFunction
+    if mesh.face_texcoords is None:
+        raise ValueError("SSS needs mesh.face_texcoords: load the mesh with Mesh.from_obj(..., load_texture=True, dr_type='softras')")
+    textures = mesh.textures
+    if textures.dim() != 4 or textures.shape[0] != 1:
+        raise ValueError("SSS supports batch size 1 with textures [1, nf, R*R, 3], got %s" % (tuple(textures.shape),))
+    dev = textures.device
+    S = int(image_size)
+    with torch.no_grad():
+        irradiance = torch.sqrt(textures * diffuseLight)
+        rasterize = SoftRasterizeFunction(image_size=S, background_color=[0, 0, 0], near=1, far=100,
+                                          fill_back=True, eps=1e-5, sigma_val=1e-5, dist_func='barycentric', dist_eps=1e-5,
+                                          gamma_val=1e-4, aggr_func_rgb='hard', aggr_func_alpha='prod', texture_type='surface')
+        # (face_vertices + 1) / 2 * 255 has T = 3 texels, so R = int(sqrt(3)) = 1 and every face samples texel 0, its
+        # vertex 0: the same map comes from that one texel
+        world = ((mesh.face_vertices + 1) / 2 * 255.)[:, :, :1].contiguous()
+        coords = (mesh.face_texcoords.to(device=dev, dtype=torch.float32) - 0.5) * 2
+        coords = torch.cat([coords, torch.full(coords.shape[:3] + (1,), 1.5, device=dev)], dim=3).contiguous()
+        final = sss_blur_chain(*[rasterize(coords, t.contiguous())[0] for t in (world, irradiance, specular)])
+        nf, T = textures.shape[1], mesh.texture_res ** 2
+        out = bake_textures_for_softras(final, mesh.face_texcoords[0], torch.ones((nf, T, 3), device=dev),
+                                        torch.ones((nf,), dtype=torch.int32, device=dev), device=dev)
+    return out[None]
+
+
+def sss_blur_chain(worldcoord_map, irradiance_map, specular_map):
+    """The image-space part of SSS (b200r_sss_blur_chain): three texture-space maps [4 (or 3), S, S] float32 on one CUDA
+    device -> the scattered colour map [S, S, 3], flipped vertically for the bake."""
+    maps = [m.contiguous() for m in (worldcoord_map, irradiance_map, specular_map)]
+    dev = maps[0].device
+    S = maps[0].shape[-1]
+    for m in maps:
+        if not m.is_cuda or m.device != dev or m.dtype != torch.float32 or m.dim() != 3 or m.shape[0] < 3 or tuple(m.shape[1:]) != (S, S):
+            raise ValueError("sss_blur_chain: three float32 CUDA maps [>=3, S, S] on one device")
+    L = _lib.lib()
+    final = torch.empty((S, S, 3), dtype=torch.float32, device=dev)
+    ws_bytes = L.b200r_sss_workspace_bytes(S)
+    workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    taps, widths, weights = _sss_host_arrays()
+    p = lambda t: C.c_void_p(t.data_ptr())   # noqa: E731
+    with torch.cuda.device(dev):
+        _lib.check(L.b200r_sss_blur_chain(p(maps[0]), p(maps[1]), p(maps[2]), p(final), p(workspace), ws_bytes, S,
+                                          taps, widths, weights, C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
+                   "b200r_sss_blur_chain")
+    return final
+
+
+def sss_blur(image, modulate, variance, dim):
+    """One stretch-modulated 7-tap blur of an [S, S] float32 CUDA map (_blur_for_SSS, gaussian_blur.py:34-165): dim 1 along
+    x, dim 0 along y, Gauss width sqrt(variance) scaled per pixel by modulate.  The building block of SSS's chain."""
+    if not (image.is_cuda and modulate.is_cuda and image.device == modulate.device):
+        raise _lib.B200RasterError("sss_blur runs on the GPU (b200r_sss_blur); there is no CPU fallback")
+    if image.dtype != torch.float32 or modulate.dtype != torch.float32:
+        raise TypeError("sss_blur: image and modulate must be float32")
+    if image.dim() != 2 or image.shape[0] != image.shape[1] or modulate.shape != image.shape:
+        raise ValueError("sss_blur: image and modulate must be the same square [S, S] map")
+    taps, w = _sss_taps(float(variance))
+    img, mod = image.contiguous(), modulate.contiguous()
+    out = torch.empty_like(img)
+    dev = img.device
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().b200r_sss_blur(C.c_void_p(img.data_ptr()), C.c_void_p(mod.data_ptr()), C.c_void_p(out.data_ptr()),
+                                             img.shape[0], (C.c_float * _SSS_TAP_NUM)(*taps), w, int(dim),
+                                             C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "b200r_sss_blur")
+    return out
+
+
 def _normalized_direction(d):
     """F.normalize(light_direction, dim=0, eps=1e-12) on the host, in float32 like the mirror."""
     t = torch.tensor([float(x) for x in (d.detach().cpu().tolist() if isinstance(d, torch.Tensor) else d)], dtype=torch.float32)
@@ -261,7 +364,8 @@ class Lighting(nn.Module):
     def forward(self, mesh, eyes=None):
         if self.Gbuffer == "albedo":
             return mesh
-        if self.light_mode == 'surface' and self._fusable(mesh, eyes):
+        sss = self.light_mode == 'surface' and mesh.textures.dim() == 4 and mesh.with_SSS
+        if self.light_mode == 'surface' and not sss and self._fusable(mesh, eyes):
             lit = self._fused_surface(mesh, eyes)
             if lit is not None:
                 mesh.textures = lit
@@ -276,7 +380,9 @@ class Lighting(nn.Module):
                     mesh.with_specular, mesh.metallic_textures, mesh.roughness_textures)
             diffuseLight = diffuseLight[:, :, None, :]
             specularLight = specularLight[:, :, None, :]
-            if mesh.textures.dim() == 4:
+            if sss:   # the fused kernel returns only diffuse and specular combined: SSS needs them apart
+                mesh.textures = torch.clamp(SSS(diffuseLight, specularLight, mesh), 0.0, 1.0)
+            elif mesh.textures.dim() == 4:
                 mesh.textures = torch.clamp(mesh.textures * diffuseLight + torch.ones_like(mesh.textures) * specularLight, 0.0, 1.0)
             elif mesh.textures.dim() == 6:
                 mesh.textures = torch.clamp(mesh.textures * diffuseLight[:, :, :, None, None, :] +

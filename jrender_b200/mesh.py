@@ -2,8 +2,9 @@
 
 Holds vertices [B,nv,3], faces [B,nf,3] and textures; lazily gathers face_vertices
 [B,nf,3,3] / face_textures -- the two tensors the rasterizer consumes.  Only the attributes the
-rasterizer path (Renderer -> Lighting -> Transform -> rasterizer) reads are mirrored; normal
-maps / TBN / SSS / voxelize are outside the hot-path scope (SURVEY.md section 8).
+rasterizer path (Renderer -> Lighting -> Transform -> rasterizer) reads are mirrored, plus the UV triangles
+(face_texcoords) that texture-space subsurface scattering (with_SSS) rasterizes; normal maps / TBN / voxelize are
+outside the hot-path scope (SURVEY.md section 8).
 """
 import numpy as np
 import torch
@@ -54,6 +55,10 @@ class Mesh(object):
         self._vertex_normals_update = True
         self._with_specular = True   # mesh.py:74: lighting takes the Cook-Torrance branch by default
         self._with_SSS = with_SSS
+        if isinstance(face_texcoords, np.ndarray):
+            face_texcoords = torch.from_numpy(face_texcoords).float()
+        if face_texcoords is not None and face_texcoords.dim() == 3:   # [nf, 3, 2] -> [1, nf, 3, 2] (mesh.py:77-79)
+            face_texcoords = face_texcoords[None]
         self._face_texcoords = face_texcoords
         self._fill_back = False
         self.dr_type = dr_type
@@ -219,15 +224,19 @@ class Mesh(object):
     @classmethod
     def from_obj(cls, filename_obj, normalization=False, load_texture=False, dr_type='softras', texture_res=1,
                  texture_type='surface', texture_wrapping='REPEAT', use_bilinear=True, with_SSS=False):
-        from .io import load_obj
+        from .io import load_obj, _parse_texture_faces
+        face_texcoords = None
         if load_texture:
             vertices, faces, textures = load_obj(filename_obj, normalization=normalization, texture_res=texture_res,
                                                  load_texture=True, dr_type=dr_type, texture_type=texture_type,
                                                  texture_wrapping=texture_wrapping, use_bilinear=use_bilinear)
+            if dr_type == 'softras' and texture_type == 'surface':   # _load_obj_for_softras.py returns the UVs too
+                face_texcoords = torch.from_numpy(_parse_texture_faces(filename_obj)[0]).to(vertices.device)
         else:
             vertices, faces = load_obj(filename_obj, normalization=normalization, load_texture=False, dr_type=dr_type)
             textures = None
-        return cls(vertices, faces, textures, texture_res, texture_type, dr_type=dr_type, with_SSS=with_SSS)
+        return cls(vertices, faces, textures, texture_res, texture_type, dr_type=dr_type, with_SSS=with_SSS,
+                   face_texcoords=face_texcoords)
 
     def save_obj(self, filename_obj, save_texture=False, texture_res_out=16):
         """structures/mesh.py:330-338.  Geometry only: the texture-atlas export (io/save_obj.py:9-29, a separate CUDA
@@ -246,6 +255,8 @@ class Mesh(object):
         self._textures = self._textures.to(device)
         self.metallic_textures = self.metallic_textures.to(device)
         self.roughness_textures = self.roughness_textures.to(device)
+        if self._face_texcoords is not None:
+            self._face_texcoords = self._face_texcoords.to(device)
         self._origin_vertices, self._origin_faces, self._origin_textures = self._vertices, self._faces, self._textures
         self._face_vertices_update = self._surface_normals_update = self._vertex_normals_update = True
         return self
